@@ -2,6 +2,7 @@
 """Benchmark of the audio template-matching hot path (BASELINE.json metric: subtitle events/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload config3]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic subtitle events: broadcast of the two
 normalised streams to every rank, stream preparation (running sums + the block spectra a rank's events
@@ -27,6 +28,10 @@ Numbers printed (one JSON line, rank 0):
           medians, normalise, running sums), per-kernel GB/s against the HBM peak, the oracle loader beside it
 
 --impl reference times the CPU path as the reference arm.
+
+--dump-outputs DIR writes what the last device-timed step computed, as find_batch returns it to a caller:
+DIR/diffs.npy (float32, one per event) and DIR/times.npy (float64 seconds).  The inputs derive from fixed seeds,
+so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -500,6 +505,11 @@ def run_b200(args):
     launches = int(lib.sb_launch_count())
     prof = profile_snapshot(lib)
     ms_total = comm.max_over_ranks([ms.value])[0]
+    if root and args.dump_outputs:
+        diff, idx = matcher.gather_results()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, 'diffs.npy'), diff)
+        np.save(os.path.join(args.dump_outputs, 'times.npy'), plan['t0'] + idx / float(SAMPLE_RATE))
 
     # ---- e2e: host buffers on the root, public API, results back on the host; wall clock bracketed by
     # barriers + device syncs, maximum over ranks
@@ -652,7 +662,12 @@ def main():
     ap.add_argument('--hop-mode', type=int, default=-1, help='fused engine geometry: 1 hop B (default), 2 hop B/2, 0 cost rule per batch')
     ap.add_argument('--epilogue', type=int, default=0, help='body variant of the packed kernels on uint8 streams: 3 run-level bounds + k_finish_runs (default), 1 first version')
     ap.add_argument('--engine', type=int, default=-1, help='0: cuFFT pipeline, 1: fused kernel, 2: packed fused kernels (default), 4 / 5: always / never pairs of lag blocks')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the results of the last timed step to DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl == 'reference' or args.load_only):
+        ap.error('--dump-outputs needs the timed matcher steps (--impl b200 without --load-only)')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
-"""Generate tests/golden/*.npz by running THE REFERENCE ITSELF (read-only at /root/reference)
-under Python 3 in this container.  TEST INFRASTRUCTURE ONLY; run here, never on the GPU box
-(/root/reference does not exist there) -- the frozen outputs travel instead.
+"""Generate tests/golden/*.npz by running THE REFERENCE ITSELF (a read-only checkout of tp7/Sushi)
+under Python 3.  TEST INFRASTRUCTURE ONLY: the tests never need the reference, the frozen outputs
+stand in for it.  Seeded inputs are stored as CRC-32s (oracle/golden_inputs.py regenerates them).
 
 What runs unmodified from the reference:
   * wav.WavStream.get_substream / find_substream / _get_sample_for_time / duration_seconds
@@ -15,7 +15,8 @@ What runs unmodified from the reference:
     mechanical py2->py3 text transform listed in PY3_EDITS below (no reference source is copied
     into this repository; the transformed text only lives in memory).
 
-Usage:  python oracle/gen_golden.py          (writes tests/golden/*.npz)
+Usage:  python oracle/gen_golden.py REFERENCE_DIR [loader|loader24|matcher|shifts ...]
+        (writes tests/golden/*.npz)
 """
 import functools
 import io
@@ -27,7 +28,9 @@ import zlib
 
 import numpy as np
 
-REF = '/root/reference'
+if len(sys.argv) < 2 or not os.path.isfile(os.path.join(sys.argv[1], 'wav.py')):
+    sys.exit(__doc__)
+REF = os.path.abspath(sys.argv[1])
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 OUT = os.path.join(ROOT, 'tests', 'golden')
@@ -39,7 +42,8 @@ import chunk as _chunk      # noqa: E402  (stdlib, still present in 3.12)
 import wav as refwav        # noqa: E402  the reference module
 import subs as refsubs      # noqa: E402
 
-from sushi_b200 import synth   # noqa: E402  seeded PCM generator (inputs only)
+from oracle import golden_inputs   # noqa: E402  seeded inputs
+from sushi_b200 import synth       # noqa: E402  seeded PCM generator (inputs only)
 
 
 class _Py2Str(bytes):
@@ -122,16 +126,9 @@ def ref_load(pcm, framerate, channels, sample_rate, sample_type, tmp='/tmp/_gold
 
 def gen_loader():
     """Loader golden: PCM in -> reference WavStream.data out, several rate/channel combinations."""
-    rng = np.random.default_rng(11)
     cases = {}
-    specs = [  # name, framerate, channels, seconds, sample_rate
-        ('mono12k', 12000, 1, 2.5, 12000),
-        ('stereo48k', 48000, 2, 1.25, 12000),
-        ('mono44k1', 44100, 1, 2.0, 12000),
-        ('stereo22k05', 22050, 2, 2.0, 12000),
-        ('mono8k_up', 8000, 1, 1.5, 12000),
-        ('six48k', 48000, 6, 0.6, 12000),
-    ]
+    inputs = golden_inputs.loader_inputs()
+    specs = golden_inputs.LOADER_SPECS
     for name, fr, ch, secs, sr in specs:
         frames = int(round(secs * fr))
         # the reference reads UNINITIALISED memory (np.empty, wav.py:119) when
@@ -140,59 +137,40 @@ def gen_loader():
         import math
         written = sum(int(round(min(fr, frames - a) * (sr / float(fr)))) for a in range(0, frames, fr))
         assert written == math.ceil(frames / float(fr) * sr), (name, written)
-        base = synth.programme_audio(frames, 100 + len(cases), rate=fr)
-        pcm = np.empty((frames, ch), np.int16)
-        for c in range(ch):
-            pcm[:, c] = np.clip(base.astype(np.int32) * (c + 2) // (ch + 1) + rng.integers(-300, 300, frames), -32768, 32767)
+        pcm = inputs[name + '_pcm']
         for st in ('uint8', 'float32'):
             s = ref_load(pcm, fr, ch, sr, st)
             cases['{0}_{1}_data'.format(name, st)] = s.data
             cases['{0}_{1}_meta'.format(name, st)] = np.array([s.sample_rate, s.sample_count, s.padding_size], np.int64)
-        cases['{0}_pcm'.format(name)] = pcm
+        cases['{0}_pcm_crc'.format(name)] = golden_inputs.crc(pcm)
         cases['{0}_spec'.format(name)] = np.array([fr, ch, sr], np.int64)
     np.savez_compressed(os.path.join(OUT, 'loader.npz'), **cases)
     print('loader.npz:', len(specs), 'cases')
 
 
-def write_wav24(path, values, framerate, channels):
-    """values: int array (frames, channels) of signed 24-bit samples -> RIFF/WAVE PCM with 3-byte samples."""
-    v = np.ascontiguousarray(values, np.int64) & 0xFFFFFF
-    raw = np.empty(v.shape + (3,), np.uint8)
-    raw[..., 0], raw[..., 1], raw[..., 2] = v & 0xFF, (v >> 8) & 0xFF, (v >> 16) & 0xFF
-    with wave.open(path, 'wb') as w:
-        w.setnchannels(channels)
-        w.setsampwidth(3)
-        w.setframerate(framerate)
-        w.writeframes(raw.tobytes())
-
-
 def gen_loader24():
     """24-bit PCM through the reference's own readframes branch (wav.py:71-74: the top 16 bits of every sample):
-    the WAV files themselves are frozen (they are small), with the reference's WavStream.data for both sample types."""
-    rng = np.random.default_rng(24)
+    the reference's WavStream.data of the seeded WAV files for both sample types."""
     cases = {}
-    for name, fr, ch, secs in (('stereo48k_24', 48000, 2, 1.25), ('mono44k1_24', 44100, 1, 2.0), ('six48k_24', 48000, 6, 0.6)):
-        frames = int(round(secs * fr))
-        base = synth.programme_audio(frames, 240 + len(cases), rate=fr).astype(np.int64)
-        vals = np.empty((frames, ch), np.int64)
-        for c in range(ch):
-            vals[:, c] = np.clip(base * 256 * (c + 2) // (ch + 1) + rng.integers(-70000, 70000, frames), -2 ** 23, 2 ** 23 - 1)
+    inputs = golden_inputs.loader24_inputs()
+    for name, *_ in golden_inputs.LOADER24_SPECS:
         tmp = '/tmp/_golden24.wav'
-        write_wav24(tmp, vals, fr, ch)
-        cases[name + '_wav'] = np.frombuffer(open(tmp, 'rb').read(), np.uint8)
+        open(tmp, 'wb').write(inputs[name + '_wav'].tobytes())
+        cases[name + '_wav_crc'] = golden_inputs.crc(inputs[name + '_wav'])
         for st in ('uint8', 'float32'):
             s = refwav.WavStream(tmp, sample_rate=12000, sample_type=st)
             cases['{0}_{1}_data'.format(name, st)] = s.data
             cases['{0}_{1}_meta'.format(name, st)] = np.array([s.sample_rate, s.sample_count, s.padding_size], np.int64)
         os.remove(tmp)
     np.savez_compressed(os.path.join(OUT, 'loader24.npz'), **cases)
-    print('loader24.npz:', len(cases) // 5, 'cases')
+    print('loader24.npz:', len(golden_inputs.LOADER24_SPECS), 'cases')
 
 
 def gen_matcher():
     """Matcher golden: reference find_substream outputs on reference-loaded streams."""
-    src_pcm, dst_pcm = synth.make_pair(24.0, 3, 1.5)
-    out = {'src_pcm': src_pcm, 'dst_pcm': dst_pcm}
+    inputs = golden_inputs.matcher_inputs()
+    src_pcm, dst_pcm = inputs['src_pcm'], inputs['dst_pcm']
+    out = {'src_pcm_crc': golden_inputs.crc(src_pcm), 'dst_pcm_crc': golden_inputs.crc(dst_pcm)}
     # (start, end, center, window) -- centre given as absolute time, like sushi.py:432,450-452
     queries = [
         (2.00, 4.50, 3.50, 1.5),      # small-window fast path (sushi.py:432)
@@ -301,7 +279,7 @@ def gen_shifts():
 
 if __name__ == '__main__':
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ['loader', 'loader24', 'matcher', 'shifts']
+    which = sys.argv[2:] or ['loader', 'loader24', 'matcher', 'shifts']
     if 'loader' in which:
         gen_loader()
     if 'loader24' in which:

@@ -8,6 +8,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+from oracle import golden_inputs  # noqa: E402
 from sushi_b200 import _hostmem  # noqa: E402
 
 _hostmem.keep_heap()
@@ -20,18 +21,18 @@ def pytest_configure(config):
 
 @pytest.fixture(scope='session')
 def golden_loader():
-    return np.load(os.path.join(GOLDEN, 'loader.npz'))
+    return golden_inputs.load(os.path.join(GOLDEN, 'loader.npz'), 'loader')
 
 
 @pytest.fixture(scope='session')
 def golden_loader24():
     """24-bit WAV files and what the reference's own loader makes of them (oracle/gen_golden.py gen_loader24)."""
-    return np.load(os.path.join(GOLDEN, 'loader24.npz'))
+    return golden_inputs.load(os.path.join(GOLDEN, 'loader24.npz'), 'loader24')
 
 
 @pytest.fixture(scope='session')
 def golden_matcher():
-    return np.load(os.path.join(GOLDEN, 'matcher.npz'))
+    return golden_inputs.load(os.path.join(GOLDEN, 'matcher.npz'), 'matcher')
 
 
 @pytest.fixture(scope='session')
